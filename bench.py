@@ -2,6 +2,7 @@
 """bench.py — IQ MSamples/s through the BLE receive hot path (demod + detect + decode).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config all|c2|c3|c5|hot]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the receive path over one batch of synthetic IQ.  The headline line is always
 BASELINE.json configs[1] ("c2"); the other configurations ride along in the same JSON line under "configs":
@@ -27,6 +28,9 @@ were gathered on rank 0 ("parity": "ok").
 `cpu_baseline` the reference's own receiver() (oracle/_ref, compiled from /root/reference) timed on this box's host
           cores on a bounded sample of the same stream.
 `--impl reference` times that CPU implementation alone (rank 0 only) on the c2 config.
+`--dump-outputs DIR` writes, after the timed steps, the c2 records of the last timed step as a caller of the receive path
+          receives them (rank 0's gathered buffer, reference order) to DIR/<field>.npy, one float64 / float32 array per record
+          field: the inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -39,6 +43,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the tree may be read-only; the benchmark writes nothing into it
 
 STREAM_INT8 = 1 << 30
 SLOT_SAMPLES = 4096
@@ -51,6 +56,7 @@ C2_WORKLOAD = ("1 GPU: single ch37 stream, 1 GiB synthetic 4 Msps int8 IQ with i
                "1 % of the bursts corrupted, 1 % placed across a chunk boundary)")
 PARITY_SLICES = 64
 PARITY_CHUNKS = 16
+DUMP_MAX_RECORDS = 200_000           # --dump-outputs: 248 B per record (float64 fields and index, float32 bytes), at most 50 MB
 
 
 def host_cores():
@@ -345,9 +351,10 @@ def parity_block(env, rx, gather, buf, d_iq, cfgs_local, stream_lo, n_streams_gl
 
 
 def run_workload(env, rx, name, d_iq, cfgs_local, stream_lo, n_streams_global, all_cfgs, n_int8, steps, warmup, bursts_local,
-                 serial_launches=0, parity_seed=1):
+                 serial_launches=0, parity_seed=1, keep_last=False):
     """Times `steps` passes over this rank's captures (double-buffered over two CUDA streams), records of all ranks
-    on rank 0 (RecordGather), then the parity block.  Returns a dict (rank 0) / partial dict (other ranks)."""
+    on rank 0 (RecordGather), then the parity block.  Returns a dict (rank 0) / partial dict (other ranks); with
+    `keep_last`, rank 0's dict holds the records of the last timed step under "last_records"."""
     import numpy as np
     from btle_b200.dist import RecordGather
     torch = env.torch
@@ -393,6 +400,11 @@ def run_workload(env, rx, name, d_iq, cfgs_local, stream_lo, n_streams_global, a
     sampler.join()
     ms_step = env.max_over_ranks(ev0.elapsed_time(ev1)) / steps
     last = (steps - 1) & 1
+    last_records = None
+    if keep_last and env.rank == 0:                # before the serial launches below reuse the buffers
+        from btle_b200.dist import shard_range
+        last_records = gather.ordered(last, [shard_range(n_streams_global, env.world, r)[0] for r in range(env.world)],
+                                      n_units=units_max)
     n_found_local = int(gather.target(last)[1][:max(units, 1), 1].sum().item()) if units else 0
     n_found = env.sum_over_ranks(n_found_local)
     n_samples = env.sum_over_ranks(n_samples_local)
@@ -419,7 +431,7 @@ def run_workload(env, rx, name, d_iq, cfgs_local, stream_lo, n_streams_global, a
     par = parity_block(env, rx, gather, last, d_iq, cfgs_local, stream_lo, n_streams_global, all_cfgs, n_int8, units_max, parity_seed)
     res = {"name": name, "ms_per_step": ms_step, "n_found": n_found, "n_found_local": n_found_local, "n_samples": n_samples,
            "n_samples_local": n_samples_local, "units": units, "cap": cap, "gather_mode": gather.mode, "serial": serial,
-           "launches_per_step": launches_per_step, "clocks": sampler.result()}
+           "launches_per_step": launches_per_step, "clocks": sampler.result(), "last_records": last_records}
     if env.rank == 0:
         parity, recs = par
         res["parity"] = parity
@@ -429,6 +441,24 @@ def run_workload(env, rx, name, d_iq, cfgs_local, stream_lo, n_streams_global, a
             res["records_on_rank0_per_rank"] = gather.counts(last, units_max)
     del gather
     return res
+
+
+def dump_records(out_dir, recs):
+    """The records as float arrays, one file per field (record i is row i of every file); more than DUMP_MAX_RECORDS
+    records are thinned to a fixed, seeded, sorted sample: index.npy holds each row's position in the full output,
+    total.npy the number of records."""
+    import numpy as np
+    total = len(recs)
+    idx = np.arange(total)
+    if total > DUMP_MAX_RECORDS:
+        idx = np.sort(np.random.default_rng(0).choice(len(recs), DUMP_MAX_RECORDS, replace=False))
+    recs = recs[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"index": idx.astype(np.float64), "total": np.array([total], dtype=np.float64)}
+    for f in recs.dtype.names:
+        arrays[f] = recs[f].astype(np.float32 if f == "bytes" else np.float64)
+    for f, a in arrays.items():
+        np.save(os.path.join(out_dir, f + ".npy"), a)
 
 
 def roofline_of(res, peak, peak_src, launch_ms=None):
@@ -452,7 +482,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true", help="kernel experiments only: the JSON line is then not a valid bench line")
     ap.add_argument("--c5-streams", type=int, default=4096, help="(experiments) number of c5 streams; BASELINE.json says 4096")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the c2 records of the last timed step to DIR/<field>.npy (float64 / float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
@@ -477,7 +511,9 @@ def main():
     cfg1 = make_cfgs(1, channel=37)
     all_cfgs = make_cfgs(world, channel=37)
     c2 = run_workload(env, rx, "c2", d_iq, cfg1, rank, world, all_cfgs, STREAM_INT8, args.steps, args.warmup, n_bursts,
-                      serial_launches=max(args.steps, 50), parity_seed=2)
+                      serial_launches=max(args.steps, 50), parity_seed=2, keep_last=bool(args.dump_outputs))
+    if rank == 0 and args.dump_outputs:
+        dump_records(args.dump_outputs, c2.pop("last_records"))
     n_samples_rank = (STREAM_INT8 // 16384) * 8192
     value = c2["n_samples"] / (c2["ms_per_step"] * 1e-3) / 1e6
     expect_ok = int((~truth["corrupt"]).sum())

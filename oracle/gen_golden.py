@@ -26,7 +26,7 @@ REF_TX = os.path.join(ROOT, "oracle", "_ref", "btle_ref_tx")
 
 
 def ref_records(iq, **cfg):
-    r = orc.ref_rx_stream(iq, **cfg)
+    r = orc.ref_rx_stream(iq, live=True, **cfg)
     return dict(exp_chunk=r["chunk"], exp_n0=r["n0"], exp_nbytes=r["nbytes"], exp_crc_bad=r["crc_bad"],
                 exp_bytes=r["bytes"])
 
@@ -60,7 +60,7 @@ def main():
     txt = open(os.path.join(REF, "matlab", "sample_iq_4msps.txt")).read()
     full = np.array([int(x) for x in re.findall(r"-?\d+", txt)], dtype=np.int8)
     assert full.size == 2097152
-    rfull = orc.ref_rx_stream(full)
+    rfull = orc.ref_rx_stream(full, live=True)
     assert list(rfull["chunk"].astype(np.int64) * 8192 + rfull["n0"]) == [97892, 501906, 905891]
     parts = [full[16384 * (k - 1):16384 * (k + 2)] for k in (11, 61, 110)]
     save("fixture_ch37.npz", np.concatenate(parts), dict(channel=37),

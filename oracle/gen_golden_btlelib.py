@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Golden vectors for the btlelib-compatible shim, produced by importing the REFERENCE's own
 python/btlelib.py here (from a writable copy: it writes table files next to itself on first TX
-call, btlelib.py:90-91,155).  Writes tests/golden/btlelib_rx.npz (committed)."""
+call, btlelib.py:90-91,155).  Writes tests/golden/btlelib_rx.npz and tests/golden/btlelib_random.npz (committed)."""
+import hashlib
 import os
 import shutil
 import sys
@@ -72,6 +73,47 @@ def main():
     out["leaf_i16"], out["leaf_q16"], out["leaf_gfsk_bit"], out["leaf_gfsk_sig"] = i16, q16, b, s
     out["hex_bits"] = bl.hex_string_to_bit("D6BE898E")
     np.savez_compressed(os.path.join(ROOT, "tests", "golden", "btlelib_rx.npz"), **out)
+    random_packets(bl)
+
+
+def random_packets(bl):
+    """60 random packets through the reference's btle_tx + add_noise at SNR 4..20 dB, cut at an arbitrary alignment, and
+    what its btle_rx made of each.  Stored: the transmitter's PHY bits and the noise parameters (the window is rebuilt by
+    tests/test_oracle_btlelib_port.py: our 8-sps modulator, which equals btle_tx's waveform, plus the seeded noise), a
+    digest of the int16 window, btle_rx's results."""
+    import torch
+    sys.path.insert(0, ROOT)
+    from btle_b200 import synth
+    cols = {f: [] for f in ("ch", "crc_hex", "aa_hex", "snr", "pad", "phy_bit", "sha256", "pdu_bit", "crc_ok", "plen", "phase")}
+    rng = np.random.default_rng(5)
+    for k in range(60):
+        ch = int(rng.choice([37, 38, 39, 3, 20]))
+        adv = ch >= 37
+        plen = int(rng.integers(6, 38)) if adv else int(rng.integers(0, 28))
+        pdu = bytes([int(rng.integers(0, 16)), plen]) + rng.integers(0, 256, plen, dtype=np.uint8).tobytes()
+        crc_hex, aa_hex = ("", "") if adv else ("A77B22", "1B0A8560")
+        pdu_bit = bl.hex_string_to_bit(pdu.hex())
+        args = [ch] + ([bl.hex_string_to_bit(crc_hex), aa_hex] if crc_hex else [])
+        ti, tq, phy_bit, _ = bl.btle_tx(pdu_bit, *args)
+        phy_bit = np.asarray(phy_bit, dtype=np.uint8)
+        mi, mq = synth.modulate_batch_8sps(torch.from_numpy(phy_bit[None, :]))
+        assert np.array_equal(mi[0].numpy(), ti) and np.array_equal(mq[0].numpy(), tq)
+        np.random.seed(100 + k)
+        snr = float(rng.choice([4.0, 7.0, 9.0, 12.0, 20.0]))
+        ri, rq = bl.add_noise(ti, tq, snr)
+        pad = int(rng.integers(0, 5)) * 8 + int(rng.integers(0, 8))          # arbitrary alignment, like a window cut from a stream
+        ri = np.concatenate((np.random.normal(0, 3, pad), ri, np.random.normal(0, 3, 64)))
+        rq = np.concatenate((np.random.normal(0, 3, pad), rq, np.random.normal(0, 3, 64)))
+        ri, rq = ri[: len(ri) // 8 * 8], rq[: len(rq) // 8 * 8]
+        r = bl.btle_rx(ri, rq, *args)
+        for f, v in (("ch", ch), ("crc_hex", crc_hex), ("aa_hex", aa_hex), ("snr", snr), ("pad", pad), ("phy_bit", phy_bit),
+                     ("sha256", hashlib.sha256(np.int16(ri).tobytes() + np.int16(rq).tobytes()).hexdigest()),
+                     ("pdu_bit", np.asarray(r[0], dtype=np.int8)), ("crc_ok", bool(r[1])), ("plen", int(r[2])), ("phase", int(r[6]))):
+            cols[f].append(v)
+    out = {f: np.array(v) for f, v in cols.items() if f not in ("phy_bit", "pdu_bit")}
+    for f in ("phy_bit", "pdu_bit"):                    # ragged: concatenated, with the end offset of each case
+        out[f], out[f + "_end"] = np.concatenate(cols[f]), np.cumsum([len(v) for v in cols[f]])
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "btlelib_random.npz"), **out)
 
 
 if __name__ == "__main__":

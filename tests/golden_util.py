@@ -9,7 +9,7 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 def cases():
     return sorted(os.path.basename(p) for p in glob.glob(os.path.join(GOLD, "*.npz"))
-                  if not os.path.basename(p).startswith("btlelib"))
+                  if not os.path.basename(p).startswith(("btlelib", "ref_driver")))
 
 
 def load(name):

@@ -3,7 +3,9 @@ oracle/_ref/btle_ref_driver = the unmodified reference receiver).  Only tests,
 __graft_entry__.smoke() and bench.py's CPU-baseline legs may import this."""
 from __future__ import annotations
 
+import atexit
 import ctypes
+import hashlib
 import os
 import subprocess
 import tempfile
@@ -86,15 +88,72 @@ def ref_available() -> bool:
     return os.path.exists(REF_DRIVER)
 
 
+# What btle_ref_driver printed and wrote, recorded once per (arguments, input contents) so that the comparisons with the
+# reference run wherever the tests run, without the reference sources.  Re-record (where oracle/_ref is built, on a
+# machine with a GPU so that the CLI cases run) with
+#     BTLE_REF_RECORD=/tmp/ref_driver.npz python -m pytest tests   and copy the file over REF_GOLDEN.
+REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_driver.npz")
+_RECORD_TO = os.environ.get("BTLE_REF_RECORD")
+_recorded = {}
+_golden = None
+
+
+def _case_key(args, inputs, outputs):
+    """Digest of the driver's arguments (paths replaced by their role) and of the contents of its inputs."""
+    h = hashlib.sha256()
+    names = {p: f"<in{i}>" for i, p in enumerate(inputs)}
+    names.update({p: f"<out{i}>" for i, p in enumerate(outputs)})
+    for a in args:
+        h.update(names.get(a, a).encode() + b"\0")
+    for p in inputs:
+        files = [os.path.join(p, f) for f in sorted(os.listdir(p))] if os.path.isdir(p) else [p]
+        for f in files:
+            h.update(os.path.basename(f).encode() + b"\0")
+            with open(f, "rb") as fh:
+                h.update(hashlib.sha256(fh.read()).digest())
+    return h.hexdigest()[:32]
+
+
+def _save_recorded():
+    old = dict(np.load(_RECORD_TO)) if os.path.exists(_RECORD_TO) else {}
+    old.update(_recorded)
+    np.savez_compressed(_RECORD_TO, **old)
+
+
+def ref_driver(args, inputs=(), outputs=(), live=False, stdout=True) -> str:
+    """btle_ref_driver (the unmodified reference) with `args` -> its stdout (if `stdout`); the files it writes land at
+    `outputs`.  `inputs` are the files / directories among `args` it reads.  Served from REF_GOLDEN unless `live` or recording."""
+    args, inputs, outputs = [str(a) for a in args], [str(p) for p in inputs], [str(p) for p in outputs]
+    key = _case_key(args, inputs, outputs)
+    if live or _RECORD_TO:
+        p = subprocess.run([REF_DRIVER] + args, check=True, capture_output=True)
+        if _RECORD_TO and not live:
+            if not _recorded:
+                atexit.register(_save_recorded)
+            _recorded[key + ".stdout"] = np.frombuffer(p.stdout if stdout else b"", dtype=np.uint8)
+            for i, o in enumerate(outputs):
+                _recorded[f"{key}.out{i}"] = np.fromfile(o, dtype=np.uint8)
+        return p.stdout.decode()
+    global _golden
+    if _golden is None:
+        _golden = np.load(REF_GOLDEN)
+    assert key + ".stdout" in _golden.files, (
+        f"no recorded reference output for btle_ref_driver {' '.join(args[:1])} on this input (case {key}): the test's input "
+        f"or arguments changed; re-record {os.path.relpath(REF_GOLDEN, ROOT)} (see tests/orc.py)")
+    for i, o in enumerate(outputs):
+        _golden[f"{key}.out{i}"].tofile(o)
+    return _golden[key + ".stdout"].tobytes().decode()
+
+
 def ref_rx_stream(iq: np.ndarray, channel=37, access_addr=0x8E89BED6, access_mask=0xFFFFFFFF, crc_init=0x555555,
-                  raw=0) -> np.ndarray:
+                  raw=0, live=False) -> np.ndarray:
     """The unmodified reference receiver() over one capture -> REF_DTYPE array."""
     iq = np.ascontiguousarray(iq, dtype=np.int8)
     with tempfile.TemporaryDirectory() as td:
         fi, fo = os.path.join(td, "iq.bin"), os.path.join(td, "out.rec")
         iq.tofile(fi)
-        subprocess.run([REF_DRIVER, "run", fi, str(channel), f"{access_addr:x}", f"{crc_init:x}", f"{access_mask:x}",
-                        str(int(raw)), fo], check=True, capture_output=True)
+        ref_driver(["run", fi, str(channel), f"{access_addr:x}", f"{crc_init:x}", f"{access_mask:x}", str(int(raw)), fo],
+                   inputs=[fi], outputs=[fo], live=live, stdout=False)
         return np.fromfile(fo, dtype=REF_DTYPE)
 
 

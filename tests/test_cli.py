@@ -1,9 +1,10 @@
 """The btle_rx-compatible host program (btle_b200/btle_rx_b200): option surface and exit codes on
 the CPU; on the GPU its text / NDJSON / pcap output against the reference's own sinks
-(oracle/_ref/btle_ref_driver sinks) for the same capture, modulo time stamps."""
+(oracle/_ref/btle_ref_driver sinks, as recorded in tests/golden/ref_driver.npz) for the same capture, modulo time stamps."""
 import os
 import re
 import subprocess
+import zlib
 
 import numpy as np
 import pytest
@@ -120,10 +121,9 @@ CASES = [
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name,ch,aa,crc,extra,mk", CASES)
 def test_cli_output_equals_reference_sinks(tmp_path, name, ch, aa, crc, extra, mk):
-    rng = np.random.default_rng(hash(name) & 0xFFFF)
+    rng = np.random.default_rng(zlib.crc32(name.encode()) & 0xFFFF)      # a seed that is the same in every process
     pdus = mk(rng)
     iq = synth.make_pdu_stream(pdus, ch, aa, crc, seed=5, corrupt={1, 7})
     f = tmp_path / "iq.bin"
@@ -133,9 +133,9 @@ def test_cli_output_equals_reference_sinks(tmp_path, name, ch, aa, crc, extra, m
     assert p.returncode == 0, p.stdout + p.stderr
     fa = extra[extra.index("-F") + 1] if "-F" in extra else "-"
     ft = extra[extra.index("-T") + 1] if "-T" in extra else "-"
-    q = subprocess.run([orc.REF_DRIVER, "sinks", str(f), str(ch), f"{aa:x}", f"{crc:x}", "ffffffff", "1" if "-r" in extra else "0",
-                        "0", "1", "1", str(ref_pcap), fa, ft], capture_output=True, text=True, check=True)
-    mine, ref = _normalise_text(p.stdout), _normalise_text(q.stdout)
+    q = orc.ref_driver(["sinks", f, ch, f"{aa:x}", f"{crc:x}", "ffffffff", "1" if "-r" in extra else "0", "0", "1", "1", ref_pcap, fa, ft],
+                       inputs=[f], outputs=[ref_pcap])
+    mine, ref = _normalise_text(p.stdout), _normalise_text(q)
     assert len(ref) >= 4
     assert mine == ref
     assert _pcap_records(mine_pcap) == _pcap_records(ref_pcap)
@@ -155,7 +155,6 @@ def test_cli_sc16_input_equals_int8_input(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built")
 def test_cli_verbose_prints_the_reference_pktbad_lines(tmp_path):
     """-v: access-address hits whose ADV header length is outside 6..37 are printed as "PktBAD" and not counted
     (btle_rx.c:2291-2298).  They come back from the GPU as BTLE_REC_REJECTED records."""
@@ -169,9 +168,8 @@ def test_cli_verbose_prints_the_reference_pktbad_lines(tmp_path):
     iq.tofile(f)
     p = run(["-i", str(f), "-c", "37", "-v", "-j"])
     assert p.returncode == 0, p.stdout + p.stderr
-    q = subprocess.run([orc.REF_DRIVER, "sinks", str(f), "37", "8e89bed6", "555555", "ffffffff", "0", "0", "1", "0", "-", "-", "-", "1"],
-                       capture_output=True, text=True, check=True)
-    mine, ref = _normalise_text(p.stdout), _normalise_text(q.stdout)
+    q = orc.ref_driver(["sinks", f, "37", "8e89bed6", "555555", "ffffffff", "0", "0", "1", "0", "-", "-", "-", "1"], inputs=[f])
+    mine, ref = _normalise_text(p.stdout), _normalise_text(q)
     assert sum(l.startswith("XXXus PktBAD") for l in ref) == 3
     assert mine == ref
     quiet = run(["-i", str(f), "-c", "37", "-j"])                             # without -v: same packets, no PktBAD lines
@@ -179,7 +177,6 @@ def test_cli_verbose_prints_the_reference_pktbad_lines(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built")
 def test_cli_hop_follows_the_connection_like_the_reference(tmp_path):
     """-o over per-channel captures (--iq-dir): text lines, packet events and hop events equal what the UNMODIFIED reference
     prints when its receiver() + receiver_controller() drive a virtual radio over the same 40 captures (oracle/_ref hop)."""

@@ -1,19 +1,17 @@
-"""oracle/btlelib_port.py (numpy restatement of the reference's bit-true Python receiver) pinned to the reference: against
-the committed golden vectors everywhere, and against the imported reference btlelib itself where /root/reference exists."""
+"""oracle/btlelib_port.py (numpy restatement of the reference's bit-true Python receiver) pinned to the reference through
+golden vectors the imported reference btlelib produced (oracle/gen_golden_btlelib.py)."""
+import hashlib
 import os
-import shutil
 import sys
-import tempfile
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import btlelib_port as P  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden", "btlelib_rx.npz")
-REF = "/root/reference/python"
+GOLD_RANDOM = os.path.join(ROOT, "tests", "golden", "btlelib_random.npz")
 
 
 def _hex_le(h):            # 'A77B22' as btlelib passes it -> the -k style integer
@@ -31,44 +29,42 @@ def test_port_equals_reference_golden_vectors():
         assert np.array_equal(r["pdu_bit"], z[f"c{n}_pdu_bit"]), n
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference not mounted")
+def _noisy_window(z, k):
+    """Case k's window as the reference's btle_rx saw it: its transmitter's waveform (= our 8-sps modulator over the PHY
+    bits it sent) plus white Gaussian noise, seeded, at the case's SNR over a peak of 127 (sigma 127 / 10^(SNR/20) split
+    evenly over I and Q), behind `pad` and ahead of 64 samples of noise alone, cut to whole symbols."""
+    import torch
+    from btle_b200 import synth
+    lo = z["phy_bit_end"][k - 1] if k else 0
+    ti, tq = synth.modulate_batch_8sps(torch.from_numpy(z["phy_bit"][lo:z["phy_bit_end"][k]][None, :]))
+    np.random.seed(100 + k)
+    sigma = 127 / np.power(10, z["snr"][k] / 20) / np.sqrt(2)
+    ri = np.double(ti[0].numpy()) + np.random.normal(0, sigma, ti.shape[1])
+    rq = np.double(tq[0].numpy()) + np.random.normal(0, sigma, tq.shape[1])
+    pad = int(z["pad"][k])
+    ri = np.concatenate((np.random.normal(0, 3, pad), ri, np.random.normal(0, 3, 64)))
+    rq = np.concatenate((np.random.normal(0, 3, pad), rq, np.random.normal(0, 3, 64)))
+    return ri[: len(ri) // 8 * 8], rq[: len(rq) // 8 * 8]
+
+
 def test_port_equals_imported_reference_on_random_packets():
-    td = tempfile.mkdtemp()
-    shutil.copytree(REF, os.path.join(td, "python"))
-    os.makedirs(os.path.join(td, "verilog"))
-    cwd = os.getcwd()
-    os.chdir(os.path.join(td, "python"))
-    sys.path.insert(0, os.getcwd())
-    try:
-        import btlelib as bl
-        rng = np.random.default_rng(5)
-        n_ok = n_bad = 0
-        for k in range(60):
-            ch = int(rng.choice([37, 38, 39, 3, 20]))
-            adv = ch >= 37
-            plen = int(rng.integers(6, 38)) if adv else int(rng.integers(0, 28))
-            pdu = bytes([int(rng.integers(0, 16)), plen]) + rng.integers(0, 256, plen, dtype=np.uint8).tobytes()
-            crc_hex, aa_hex = ("", "") if adv else ("A77B22", "1B0A8560")
-            pdu_bit = bl.hex_string_to_bit(pdu.hex())
-            args = [ch] + ([bl.hex_string_to_bit(crc_hex), aa_hex] if crc_hex else [])
-            ti, tq, _, _ = bl.btle_tx(pdu_bit, *args)
-            np.random.seed(100 + k)
-            snr = float(rng.choice([4.0, 7.0, 9.0, 12.0, 20.0]))
-            ri, rq = bl.add_noise(ti, tq, snr)
-            pad = int(rng.integers(0, 5)) * 8 + int(rng.integers(0, 8))          # arbitrary alignment, like a window cut from a stream
-            ri = np.concatenate((np.random.normal(0, 3, pad), ri, np.random.normal(0, 3, 64)))
-            rq = np.concatenate((np.random.normal(0, 3, pad), rq, np.random.normal(0, 3, 64)))
-            ri, rq = ri[: len(ri) // 8 * 8], rq[: len(rq) // 8 * 8]
-            ref = bl.btle_rx(ri, rq, *args)
-            got = P.rx_window(np.int16(ri), np.int16(rq), ch, int(crc_hex, 16) if crc_hex else 0x555555,
-                              int.from_bytes(bytes.fromhex(aa_hex), "little") if aa_hex else 0x8E89BED6)
-            assert got["crc_ok"] == bool(ref[1]) and got["plen"] == int(ref[2]) and got["phase"] == int(ref[6]), (k, snr)
-            assert np.array_equal(got["pdu_bit"], np.asarray(ref[0], dtype=np.int8)), (k, snr)
-            n_ok += bool(ref[1]); n_bad += not ref[1]
-        assert n_ok > 20 and n_bad > 5
-    finally:
-        os.chdir(cwd)
-        sys.path.remove(os.path.join(td, "python"))
+    """60 random packets at SNR 4..20 dB and arbitrary alignment, against what the reference's btle_rx returned for each
+    (tests/golden/btlelib_random.npz, written by oracle/gen_golden_btlelib.py from the imported reference btlelib)."""
+    z = np.load(GOLD_RANDOM)
+    n_ok = n_bad = 0
+    for k in range(len(z["ch"])):
+        ri, rq = _noisy_window(z, k)
+        ri, rq = np.int16(ri), np.int16(rq)
+        assert hashlib.sha256(ri.tobytes() + rq.tobytes()).hexdigest() == z["sha256"][k], k       # the window the reference saw
+        crc_hex, aa_hex = str(z["crc_hex"][k]), str(z["aa_hex"][k])
+        got = P.rx_window(ri, rq, int(z["ch"][k]), int(crc_hex, 16) if crc_hex else 0x555555,
+                          int.from_bytes(bytes.fromhex(aa_hex), "little") if aa_hex else 0x8E89BED6)
+        lo = z["pdu_bit_end"][k - 1] if k else 0
+        ref_ok = bool(z["crc_ok"][k])
+        assert got["crc_ok"] == ref_ok and got["plen"] == int(z["plen"][k]) and got["phase"] == int(z["phase"][k]), (k, z["snr"][k])
+        assert np.array_equal(got["pdu_bit"], z["pdu_bit"][lo:z["pdu_bit_end"][k]]), (k, z["snr"][k])
+        n_ok += ref_ok; n_bad += not ref_ok
+    assert n_ok > 20 and n_bad > 5
 
 
 def test_port_stream_finds_what_it_sent():

@@ -1,14 +1,12 @@
-"""Pins our C restatement (oracle/btle_oracle.c) to the reference itself
-(oracle/_ref = /root/reference's btle_rx.c compiled unmodified).  Runs wherever
-oracle/_ref exists (here, and on the GPU box where the built binaries travel)."""
+"""Pins our C restatement (oracle/btle_oracle.c) to the reference itself (oracle/_ref = the reference's btle_rx.c
+compiled unmodified), through what its receiver() returned for these very inputs, recorded in tests/golden/ref_driver.npz
+(tests/orc.py: ref_driver)."""
 import numpy as np
 import pytest
 import torch
 
 import orc
 from btle_b200 import synth
-
-needs_ref = pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built")
 
 
 def _cmp(iq, **cfg):
@@ -18,7 +16,6 @@ def _cmp(iq, **cfg):
     return rec
 
 
-@needs_ref
 def test_synth_adv_stream_all_adv_channels():
     for ch in (37, 38, 39):
         iq, truth = synth.make_adv_stream(512 * 1024, seed=100 + ch, channel=ch, corrupt_every=7)
@@ -27,7 +24,6 @@ def test_synth_adv_stream_all_adv_channels():
         assert rec["crc_bad"].sum() >= 1
 
 
-@needs_ref
 def test_data_channels_custom_aa_crcinit():
     for ch in (0, 9, 10, 36):
         aa, ci = 0x60850A1B + ch, 0xA77B22 ^ ch
@@ -37,14 +33,12 @@ def test_data_channels_custom_aa_crcinit():
         assert len(rec) >= 50
 
 
-@needs_ref
 def test_raw_mode():
     iq, _ = synth.make_adv_stream(256 * 1024, seed=5, channel=37)
     rec = _cmp(iq.numpy(), channel=37, raw=1)
     assert len(rec) >= 30 and (rec["n_bytes"] == 42).all()
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(6))
 def test_fuzz_random_iq_loose_masks(seed):
     """Adversarial: full-scale random IQ with sparse masks -> very many hits, negative
@@ -61,7 +55,6 @@ def test_fuzz_random_iq_loose_masks(seed):
             assert len(rec) > 8
 
 
-@needs_ref
 def test_fuzz_small_amplitude_zero_products():
     """d uses a strict > 0 (btle_rx.c:1533): zeros and tiny amplitudes must give bit 0."""
     rng = np.random.default_rng(99)
@@ -70,7 +63,6 @@ def test_fuzz_small_amplitude_zero_products():
     _cmp(np.zeros(3 * 16384, dtype=np.int8), channel=37, access_addr=0, access_mask=0xFFFFFFFF)
 
 
-@needs_ref
 def test_short_and_ragged_lengths():
     rng = np.random.default_rng(3)
     for n in (0, 100, 16383, 16384, 16385, 16384 + 3007, 2 * 16384 + 1):
@@ -78,7 +70,6 @@ def test_short_and_ragged_lengths():
         _cmp(iq, channel=37, access_mask=0xFF)
 
 
-@needs_ref
 def test_worst_case_packets_per_chunk():
     """BTLE_MAX_PKTS_PER_CHUNK (include/btle_b200.h): with mask 0 every window matches, through the zeroed
     history up to 31 symbols before the restart point, so a zero-length data PDU advances the cursor by only

@@ -45,7 +45,7 @@ for e in extra:
     print("   decoded vs transmitted PDU (byte index, xor):", diff, "lengths", len(got), len(sent))
     if orc.ref_available():
         try:
-            orc.assert_same_as_ref(mine, orc.ref_rx_stream(host[lo:hi]))
+            orc.assert_same_as_ref(mine, orc.ref_rx_stream(host[lo:hi], live=True))
             print("   unmodified reference: equal")
         except AssertionError as ex:
             print("   unmodified reference: DIFFERENT", ex)

@@ -60,6 +60,6 @@ while time.time() - t0 < float(os.environ.get("FUZZ_SECONDS", "300")):
     uw = np.concatenate([ur[int(b):int(b) + int(c)] for b, c in ud]) if len(ud) else ur[:0]
     assert uw.tobytes() == o.tobytes(), ("emul units != oracle", kind, n, cfg)
     if orc.ref_available():
-        orc.assert_same_as_ref(o, orc.ref_rx_stream(iq, **cfg))
+        orc.assert_same_as_ref(o, orc.ref_rx_stream(iq, live=True, **cfg))
     n_case += 1; n_pkt += len(o); kinds[kind] = kinds.get(kind, 0) + len(o)
 print(f"fuzz ok: {n_case} cases, {n_pkt} packets compared, packets per input kind {kinds}, ref={'yes' if orc.ref_available() else 'no'}")
