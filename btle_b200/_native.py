@@ -38,6 +38,9 @@ BER_CFG_DTYPE = np.dtype([("seed", "<u8"), ("snr_db", "<f4"), ("ppm", "<f4"), ("
 BER_RESULT_DTYPE = np.dtype([("packets", "<u8"), ("pkt_err", "<u8"), ("bit_err", "<u8"), ("bit_total", "<u8"), ("aa_miss", "<u8"), ("seconds", "<f8")])
 assert BER_CFG_DTYPE.itemsize == 32 and BER_RESULT_DTYPE.itemsize == 48
 SPS8_REC_DTYPE = np.dtype([("sample", "<i8"), ("window", "<i8"), ("rx", MODEL_REC_DTYPE)])     # btle_sps8_rec
+# btle_wideband_cfg, 16 bytes
+WIDEBAND_CFG_DTYPE = np.dtype([("decim", "<i4"), ("center_mhz", "<i4"), ("out_shift", "<i4"), ("reserved", "<i4")])
+assert WIDEBAND_CFG_DTYPE.itemsize == 16
 assert REC_DTYPE.itemsize == 64 and CFG_DTYPE.itemsize == 24 and MODEL_REC_DTYPE.itemsize == 80 and SPS8_REC_DTYPE.itemsize == 96
 
 EXPORTS = [
@@ -53,6 +56,7 @@ EXPORTS = [
     "btle_b200_stream_close", "btle_b200_stream_set_cfg", "btle_b200_parse_adv_pdu_payload_byte", "btle_b200_parse_ll_pdu_payload_byte",
     "btle_b200_receiver_controller", "btle_b200_receiver_status", "btle_b200_note_packet", "btle_b200_set_hop_hooks", "btle_b200_hop_reset",
     "btle_b200_get_freq_by_channel_number", "btle_b200_chm_is_full_map",
+    "btle_b200_wideband_taps", "btle_b200_channelize_device", "btle_b200_channelize", "btle_b200_rx_wideband",
 ]
 
 
@@ -118,6 +122,10 @@ def load():
     L.btle_b200_sps8_hits_device.argtypes = [vp, vp, sz, u32, vp, sz, vp, vp]
     L.btle_b200_rx_sps8.argtypes = [vp, vp, sz, i32, u32, u32, vp, sz, ctypes.POINTER(sz)]
     L.btle_b200_synth_streams_device.argtypes = [vp, vp, sz, sz, sz, vp, vp, vp, sz, ctypes.POINTER(sz), vp]
+    L.btle_b200_wideband_taps.argtypes = [vp, i32, vp, sz, ctypes.POINTER(sz), ctypes.POINTER(ctypes.c_int)]
+    L.btle_b200_channelize_device.argtypes = [vp, vp, sz, vp, vp, sz, vp, sz, vp]
+    L.btle_b200_channelize.argtypes = [vp, vp, sz, vp, vp, sz, vp, sz]
+    L.btle_b200_rx_wideband.argtypes = [vp, vp, sz, vp, vp, sz, vp, sz, ctypes.POINTER(sz)]
     _lib = L
     return L
 

@@ -18,6 +18,10 @@
 //                                init, decoded in ONE batched launch; packets are printed in time order.
 //       --iq-dir DIR             DIR/ch00.bin .. DIR/ch39.bin, time-aligned captures of the BLE channels (missing
 //                                files are skipped).  Without -o: like 40 -i entries.  With -o: see below.
+//       --wideband FILE:RATE_MSPS:CENTER_MHZ   one int8 I,Q capture of the band at RATE_MSPS (a multiple of 4) centred on
+//                                CENTER_MHZ (one SDR, hackrf_transfer -r / UHD sc8): every BLE channel inside the band is
+//                                channelized on the GPU to 4 Msps (btle_b200_channelize), then handled exactly like
+//                                --iq-dir, with and without -o; time stamps are on the 4 Msps channel time base.
 //       --iq-txt FILE / --iq-sc16 FILE   text format of save_phy_sample (btle_rx.c:896-915) / int16 bladeRF samples.
 //   * -o (hop) with --iq-dir: the reference retunes its ONE radio; here a virtual radio walks the per-channel captures
 //     chunk by chunk with the reference's own state machine (btle_b200_receiver_controller == receiver_controller,
@@ -59,7 +63,7 @@ struct Options {
   int chan = 37, gain = 6, lna = 32, amp = 0, verbose = 0, raw = 0, hop = 0, json = 0, quiet = 0, rssi = 0;
   uint32_t aa = 0x8E89BED6u, crc_init = 0x555555u, mask = 0xFFFFFFFFu;
   uint64_t freq_hz = 123;
-  const char *pcap = nullptr, *iq_txt = nullptr, *iq_sc16 = nullptr, *iq_dir = nullptr, *iq_bin16 = nullptr;
+  const char *pcap = nullptr, *iq_txt = nullptr, *iq_sc16 = nullptr, *iq_dir = nullptr, *iq_bin16 = nullptr, *wideband = nullptr;
   std::vector<std::string> iq_files;            // -i, possibly FILE:CH[:AA[:CRCINIT]]
   size_t segment_chunks = 4096;
   int filter_adva_set = 0;
@@ -75,6 +79,8 @@ void usage() {
       "    -i --iq-file FILE[:CH[:AA[:CRCINIT]]]\n      raw interleaved int8 I,Q capture at 4 Msps ('-' = stdin)   [this build: no SDR]\n"
       "      repeatable: several captures are decoded in one batch, each with its own channel / access address / CRC init\n"
       "       --iq-dir DIR\n      DIR/ch00.bin .. DIR/ch39.bin (time-aligned per-channel captures); with -o the connection is followed across them\n"
+      "       --wideband FILE:RATE_MSPS:CENTER_MHZ\n      one int8 I,Q capture of the band (RATE_MSPS a multiple of 4, 8..256); every channel inside it is\n"
+      "      channelized to 4 Msps on the GPU and decoded like --iq-dir (with -o the connection is followed across them)\n"
       "       --iq-bin16 FILE\n      interleaved int16 I,Q at 8 Msps (8 samples per symbol): a `btle_ll -q` capture; decoded with the 8-phase\n"
       "      CRC-select receiver of the reference's Python / Verilog model (first sample phase whose CRC is ok wins)\n"
       "       --segment-chunks N\n      chunks (16384 int8) per streamed segment of a single capture (default 4096 = 64 MiB)\n"
@@ -135,7 +141,7 @@ Options parse_commandline(int argc, char **argv) {
       {"filter-pdu-type", required_argument, 0, 'T'}, {"iq-file", required_argument, 0, 'i'},
       {"iq-txt", required_argument, 0, 1000}, {"iq-sc16", required_argument, 0, 1001}, {"device", required_argument, 0, 'd'},
       {"iq-dir", required_argument, 0, 1002}, {"segment-chunks", required_argument, 0, 1003}, {"iq-bin16", required_argument, 0, 1004},
-      {0, 0, 0, 0}};
+      {"wideband", required_argument, 0, 1005}, {0, 0, 0, 0}};
   for (;;) {
     int idx = 0;
     const int c = getopt_long(argc, argv, "hc:g:l:ba:k:vrf:m:os:jQRF:T:i:d:", longopts, &idx);   // + i:, d:
@@ -160,6 +166,7 @@ Options parse_commandline(int argc, char **argv) {
       case 'i': o.iq_files.push_back(optarg); break;
       case 1002: o.iq_dir = optarg; break;
       case 1004: o.iq_bin16 = optarg; break;
+      case 1005: o.wideband = optarg; break;
       case 1003: o.segment_chunks = (size_t)strtoul(optarg, &endp, 10); break;
       case 1000: o.iq_txt = optarg; break;
       case 1001: o.iq_sc16 = optarg; break;
@@ -434,7 +441,45 @@ double rec_time(const btle_pkt_rec &r) { return ((double)r.chunk * 8192.0 + r.n0
 volatile sig_atomic_t g_stop = 0;
 void on_sigint(int) { g_stop = 1; }                                             // btle_rx.c:100-104
 
-struct Capture { std::string file; int chan; uint32_t aa, crc_init; };
+struct Capture { std::string file; int chan; uint32_t aa, crc_init; std::vector<int8_t> *mem = nullptr; };
+
+// a per-channel capture: the file, or (--wideband) the channel already channelized into memory
+bool load_capture(const Capture &c, std::vector<int8_t> &iq) {
+  if (c.mem) { iq.swap(*c.mem); return true; }
+  return load_raw(c.file.c_str(), iq);
+}
+
+// --wideband FILE:RATE_MSPS:CENTER_MHZ -> chan_iq[ch] = 4 Msps capture of every channel inside the band, one Capture each
+// (advertising access address / CRC init on 37..39, -a / -k elsewhere, as for --iq-dir)
+int load_wideband(btle_b200_ctx *ctx, const Options &o, std::vector<std::vector<int8_t>> &chan_iq, std::vector<Capture> &caps) {
+  const std::string spec = o.wideband;
+  const size_t c2 = spec.rfind(':'), c1 = c2 == std::string::npos || c2 == 0 ? std::string::npos : spec.rfind(':', c2 - 1);
+  char *e1 = nullptr, *e2 = nullptr;
+  const long rate = c1 == std::string::npos ? 0 : strtol(spec.c_str() + c1 + 1, &e1, 10);
+  const long center = c1 == std::string::npos ? 0 : strtol(spec.c_str() + c2 + 1, &e2, 10);
+  if (c1 == std::string::npos || *e1 != ':' || *e2 || rate < 8 || rate > 256 || rate % 4) {
+    printf("--wideband expects FILE:RATE_MSPS:CENTER_MHZ with RATE_MSPS a multiple of 4 in 8..256: %s\n", o.wideband);
+    return BTLE_EINVAL;
+  }
+  std::vector<int8_t> wide;
+  if (!load_raw(spec.substr(0, c1).c_str(), wide)) return BTLE_EINVAL;
+  const btle_wideband_cfg cfg{(int32_t)(rate / 4), (int32_t)center, -1, 0};
+  std::vector<int32_t> chans;
+  for (int ch = 0; ch < 40; ++ch)
+    if (std::labs((long)(freq_by_channel(ch) / 1000000) - center) + 1 <= 2 * cfg.decim) chans.push_back(ch);
+  if (chans.empty()) { printf("no BLE channel inside %ld Msps around %ld MHz\n", rate, center); return BTLE_EINVAL; }
+  const size_t n = wide.size() / 2, width = 2 * ((n + cfg.decim - 1) / cfg.decim), stride = (width + 15) & ~size_t(15);
+  std::vector<int8_t> out(stride * chans.size());
+  const int rc = btle_b200_channelize(ctx, wide.data(), n, &cfg, chans.data(), chans.size(), out.data(), stride);
+  if (rc) { printf("btle_b200_channelize: %s (%s)\n", btle_b200_strerror(rc), btle_b200_last_error(ctx)); return rc; }
+  for (size_t i = 0; i < chans.size(); ++i) {
+    const int ch = chans[i];
+    chan_iq[ch].assign(out.begin() + i * stride, out.begin() + i * stride + width);
+    const bool adv = ch >= 37;
+    caps.push_back(Capture{o.wideband, ch, adv ? 0x8E89BED6u : o.aa, adv ? 0x555555u : o.crc_init, &chan_iq[ch]});
+  }
+  return BTLE_OK;
+}
 
 // "FILE[:CH[:AA[:CRCINIT]]]"
 Capture parse_capture(const std::string &spec, const Options &o) {
@@ -516,7 +561,7 @@ int main(int argc, char **argv) {
     if (!sinks.pcap) { perror(o.pcap); return 1; }
   }
   if (o.json) json_status(0.0, "start", o);
-  if (o.iq_files.empty() && !o.iq_txt && !o.iq_sc16 && !o.iq_dir && !o.iq_bin16) {
+  if (o.iq_files.empty() && !o.iq_txt && !o.iq_sc16 && !o.iq_dir && !o.iq_bin16 && !o.wideband) {
     printf("open_board: no SDR support in this build; give a capture with -i/--iq-file\n");
     if (o.json) json_status(0.0, "stop", o);
     return 1;                                                                   // btle_rx.c:2586
@@ -552,6 +597,10 @@ int main(int argc, char **argv) {
     }
     if (caps.empty()) { printf("no chNN.bin capture found in %s\n", o.iq_dir); btle_b200_destroy(ctx); return 1; }
   }
+  // per-channel captures of the band: --iq-dir files or the channels of --wideband; the paths below do not tell them apart
+  std::vector<std::vector<int8_t>> wide_ch(40);
+  if (o.wideband && !o.iq_dir && load_wideband(ctx, o, wide_ch, caps) != BTLE_OK) { btle_b200_destroy(ctx); return 1; }
+  const char *per_channel = o.iq_dir ? o.iq_dir : o.wideband;
   for (const Capture &c : caps)
     if (c.chan < 0 || c.chan > 39) { printf("channel number must be within 0~%d!\n", 39); btle_b200_destroy(ctx); return 1; }
 
@@ -580,15 +629,15 @@ int main(int argc, char **argv) {
       sinks.packet(r, (double)recs[i].sample / 8.0e6);
     }
     t_end = (double)n_samples / 8.0e6;
-  } else if (o.hop && o.iq_dir) {
+  } else if (o.hop && per_channel) {
     // ---- connection following over per-channel captures ---------------------------------------------------------
     std::vector<std::vector<int8_t>> iq(40);
     size_t n = SIZE_MAX;
     for (const Capture &c : caps) {
-      if (!load_raw(c.file.c_str(), iq[c.chan])) { btle_b200_destroy(ctx); return 1; }
+      if (!load_capture(c, iq[c.chan])) { btle_b200_destroy(ctx); return 1; }
       n = std::min(n, iq[c.chan].size());
     }
-    if (iq[o.chan].empty()) { printf("no capture of the start channel %d in %s\n", o.chan, o.iq_dir); btle_b200_destroy(ctx); return 1; }
+    if (iq[o.chan].empty()) { printf("no capture of the start channel %d in %s\n", o.chan, per_channel); btle_b200_destroy(ctx); return 1; }
     const long long nchunks = (long long)(n / BTLE_CHUNK_INT8);
     HopRun run{&o};
     btle_hop_hooks hooks{hop_now, hop_set_freq, hop_event, &run, o.quiet};
@@ -652,12 +701,12 @@ int main(int argc, char **argv) {
     }
     btle_b200_set_hop_hooks(nullptr);
     t_end = (double)(n / 2) / 4.0e6;
-  } else if (caps.size() > 1 || (caps.size() == 1 && o.iq_dir)) {
+  } else if (caps.size() > 1 || (caps.size() == 1 && per_channel)) {
     // ---- several captures: one batched launch, packets in time order ------------------------------------------------
     std::vector<std::vector<int8_t>> iq(caps.size());
     size_t n = SIZE_MAX;
     for (size_t s_ = 0; s_ < caps.size(); ++s_) {
-      if (!load_raw(caps[s_].file.c_str(), iq[s_])) { btle_b200_destroy(ctx); return 1; }
+      if (!load_capture(caps[s_], iq[s_])) { btle_b200_destroy(ctx); return 1; }
       n = std::min(n, iq[s_].size());
     }
     const size_t stride = (n + 15) & ~size_t(15);

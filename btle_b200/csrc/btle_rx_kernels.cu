@@ -32,6 +32,7 @@
 #include "../../include/btle_b200.h"
 #include "btle_core.cuh"
 #include "btle_params.h"
+#include "btle_wideband.h"
 
 using namespace btle;
 
@@ -1393,6 +1394,8 @@ struct btle_b200_ctx {
   int8_t *h_stage[2] = {nullptr, nullptr}; size_t h_stage_bytes = 0;   // pinned staging for pageable callers
   cudaEvent_t stage_free[2] = {nullptr, nullptr};
   void *d_leaf = nullptr; size_t d_leaf_bytes = 0;
+  int8_t *d_wide = nullptr; size_t d_wide_bytes = 0;   // wideband capture of the host-buffer channelizer entry points
+  btle_wb::Scratch wb;
 };
 
 namespace {
@@ -1789,6 +1792,8 @@ void btle_b200_destroy(btle_b200_ctx *ctx) {
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
   cudaFree(ctx->d_iq); cudaFree(ctx->d_out); cudaFree(ctx->d_dir); cudaFree(ctx->d_count); cudaFree(ctx->d_count_ring); cudaFree(ctx->d_leaf);
+  cudaFree(ctx->d_wide);
+  btle_wb::release(&ctx->wb);
   for (CfgSlot &c : ctx->cfg_slot) { cudaFree(c.d); cudaFree(c.d_params); if (c.last_use) cudaEventDestroy(c.last_use); }
   if (ctx->h_count) cudaFreeHost(ctx->h_count);
   if (ctx->h_recs) cudaFreeHost(ctx->h_recs);
@@ -1891,6 +1896,104 @@ int btle_b200_rx_iq16(btle_b200_ctx *ctx, const int16_t *iq16, size_t n_int16, i
   rc = btle_b200_rx_device(ctx, ctx->d_iq, 1, pitch, n_int16, cfg, ctx->d_out, cap, ctx->d_count, st);
   if (rc) return rc;
   return fetch_ordered(ctx, ctx->d_out, ctx->d_dir, btle_b200_rx_units(ctx, 1, n_int16), out, cap, n_out, st);
+}
+
+// ---- wideband captures: channelizer (btle_wideband.cu) in front of the receiver -------------------------------------
+static int wideband_check(btle_b200_ctx *ctx, size_t n_samples, const btle_wideband_cfg *cfg, const int32_t *channels, size_t n_ch,
+                          size_t out_stride) {
+  if (!cfg) { ctx->err = "wideband cfg is NULL"; return BTLE_EINVAL; }
+  const int rc = btle_wb::validate(*cfg, channels, n_ch, &ctx->err);
+  if (rc) return rc;
+  if (out_stride & 15) { ctx->err = "channel output stride must be a multiple of 16"; return BTLE_EINVAL; }
+  if (n_ch && out_stride < 2 * btle_wb::out_samples(n_samples, cfg->decim)) {
+    ctx->err = "channel output stride " + std::to_string(out_stride) + " is smaller than 2*ceil(n_samples/decim) = " +
+               std::to_string(2 * btle_wb::out_samples(n_samples, cfg->decim));
+    return BTLE_EINVAL;
+  }
+  return BTLE_OK;
+}
+
+// host capture -> context scratch (d_wide) -> channels in ctx->d_iq, rows of out_stride bytes; enqueued on `st`
+static int wideband_stage(btle_b200_ctx *ctx, const int8_t *wide, size_t n_samples, const btle_wideband_cfg &cfg, const int32_t *channels,
+                          size_t n_ch, size_t out_stride, cudaStream_t st) {
+  int rc = ensure(ctx, reinterpret_cast<void **>(&ctx->d_wide), &ctx->d_wide_bytes, std::max<size_t>(2 * n_samples, 16));
+  if (rc) return rc;
+  rc = ensure(ctx, reinterpret_cast<void **>(&ctx->d_iq), &ctx->d_iq_bytes, std::max<size_t>(n_ch * out_stride, 16));
+  if (rc) return rc;
+  rc = h2d_rows(ctx, ctx->d_wide, 2 * n_samples, wide, 2 * n_samples, 2 * n_samples, 1, st);
+  if (rc) return rc;
+  return btle_wb::launch(&ctx->wb, ctx->d_wide, n_samples, cfg, channels, n_ch, ctx->d_iq, out_stride, st, &ctx->err);
+}
+
+int btle_b200_wideband_taps(const btle_wideband_cfg *cfg, int channel, int16_t *taps, size_t cap, size_t *n_taps, int *out_shift) {
+  if (!cfg || !n_taps || (!taps && cap)) return BTLE_EINVAL;
+  std::string err;
+  std::vector<int16_t> h;
+  int shift = 0;
+  const int rc = btle_wb::channel_taps(*cfg, channel, &h, &shift, &err);
+  if (rc) return rc;
+  *n_taps = h.size() / 2;
+  if (out_shift) *out_shift = shift;
+  if (cap < *n_taps) return BTLE_EOVERFLOW;
+  memcpy(taps, h.data(), h.size() * sizeof(int16_t));
+  return BTLE_OK;
+}
+
+int btle_b200_channelize_device(btle_b200_ctx *ctx, const int8_t *d_wide, size_t n_samples, const btle_wideband_cfg *cfg,
+                                const int32_t *channels, size_t n_ch, int8_t *d_out, size_t out_stride, void *cuda_stream) {
+  if (!ctx) return BTLE_EINVAL;
+  int rc = wideband_check(ctx, n_samples, cfg, channels, n_ch, out_stride);
+  if (rc) return rc;
+  if ((!d_wide && n_samples) || (!d_out && n_ch)) { ctx->err = "device buffer is NULL"; return BTLE_EINVAL; }
+  if ((reinterpret_cast<uintptr_t>(d_wide) & 15) || (reinterpret_cast<uintptr_t>(d_out) & 15)) {
+    ctx->err = "device wideband input and channel output must be 16-byte aligned";
+    return BTLE_EINVAL;
+  }
+  BTLE_CUDA(ctx, cudaSetDevice(ctx->device));
+  return btle_wb::launch(&ctx->wb, d_wide, n_samples, *cfg, channels, n_ch, d_out, out_stride, reinterpret_cast<cudaStream_t>(cuda_stream),
+                         &ctx->err);
+}
+
+int btle_b200_channelize(btle_b200_ctx *ctx, const int8_t *wide, size_t n_samples, const btle_wideband_cfg *cfg, const int32_t *channels,
+                         size_t n_ch, int8_t *out, size_t out_stride) {
+  if (!ctx) return BTLE_EINVAL;
+  int rc = wideband_check(ctx, n_samples, cfg, channels, n_ch, out_stride);
+  if (rc) return rc;
+  if ((!wide && n_samples) || (!out && n_ch)) { ctx->err = "host buffer is NULL"; return BTLE_EINVAL; }
+  if (!n_ch || !n_samples) return BTLE_OK;
+  BTLE_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  rc = wideband_stage(ctx, wide, n_samples, *cfg, channels, n_ch, out_stride, st);
+  if (rc) return rc;
+  const size_t width = 2 * btle_wb::out_samples(n_samples, cfg->decim);   // the padding of each row is left as it is
+  BTLE_CUDA(ctx, cudaMemcpy2DAsync(out, out_stride, ctx->d_iq, out_stride, width, n_ch, cudaMemcpyDeviceToHost, st));
+  BTLE_CUDA(ctx, cudaStreamSynchronize(st));
+  return BTLE_OK;
+}
+
+int btle_b200_rx_wideband(btle_b200_ctx *ctx, const int8_t *wide, size_t n_samples, const btle_wideband_cfg *cfg,
+                          const btle_stream_cfg *cfgs, size_t n_ch, btle_pkt_rec *out, size_t cap, size_t *n_out) {
+  if (!ctx || !n_out || (!out && cap) || (!cfgs && n_ch) || (!wide && n_samples)) return BTLE_EINVAL;
+  *n_out = 0;
+  if (!cfg) { ctx->err = "wideband cfg is NULL"; return BTLE_EINVAL; }
+  std::vector<int32_t> channels(n_ch);
+  for (size_t i = 0; i < n_ch; ++i) channels[i] = cfgs[i].channel;
+  const size_t n_int8 = 2 * btle_wb::out_samples(n_samples, std::max(cfg->decim, 1)), stride = (n_int8 + 15) & ~size_t(15);
+  int rc = wideband_check(ctx, n_samples, cfg, channels.data(), n_ch, stride);
+  if (rc) return rc;
+  BTLE_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  size_t out_bytes = ctx->d_out_cap * sizeof(btle_pkt_rec);
+  rc = ensure(ctx, reinterpret_cast<void **>(&ctx->d_out), &out_bytes, std::max<size_t>(cap, 1) * sizeof(btle_pkt_rec));
+  ctx->d_out_cap = out_bytes / sizeof(btle_pkt_rec);
+  if (rc) return rc;
+  if (n_ch && n_samples) {
+    rc = wideband_stage(ctx, wide, n_samples, *cfg, channels.data(), n_ch, stride, st);
+    if (rc) return rc;
+  }
+  rc = btle_b200_rx_device(ctx, ctx->d_iq, n_ch, stride, n_int8, cfgs, ctx->d_out, cap, ctx->d_count, st);
+  if (rc) return rc;
+  return fetch_ordered(ctx, ctx->d_out, ctx->d_dir, btle_b200_rx_units(ctx, n_ch, n_int8), out, cap, n_out, st);
 }
 
 int btle_b200_rx(btle_b200_ctx *ctx, const int8_t *iq, size_t n_int8, const btle_stream_cfg *cfg, btle_pkt_rec *out,

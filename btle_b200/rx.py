@@ -11,7 +11,7 @@ import ctypes
 import numpy as np
 
 from . import _native
-from ._native import BTLE_EOVERFLOW, BtleError, CFG_DTYPE, DIR_DTYPE, REC_DTYPE
+from ._native import BTLE_EINVAL, BTLE_EOVERFLOW, BtleError, CFG_DTYPE, DIR_DTYPE, REC_DTYPE, WIDEBAND_CFG_DTYPE
 
 DEFAULT_ACCESS_ADDR = 0x8E89BED6     # btle_rx.c:231
 DEFAULT_CRC_INIT = 0x555555          # btle_rx.c:232
@@ -25,6 +25,35 @@ def make_cfgs(n_streams=1, channel=DEFAULT_CHANNEL, access_addr=DEFAULT_ACCESS_A
     c["channel"], c["access_addr"], c["access_mask"] = channel, access_addr, access_mask
     c["crc_init"], c["raw"], c["rssi"] = crc_init, raw, rssi
     return c
+
+
+def _wideband_cfg(decim: int, center_mhz: int, out_shift: int = -1) -> np.ndarray:
+    c = np.zeros(1, dtype=WIDEBAND_CFG_DTYPE)
+    c["decim"], c["center_mhz"], c["out_shift"] = decim, center_mhz, out_shift
+    return c
+
+
+def band_channels(decim: int, center_mhz: int) -> list:
+    """The BLE channels inside a capture at 4 MHz * decim centred on center_mhz (|f_ch - fc| + 1 MHz <= fs / 2)."""
+    from .hop import channel_freq_mhz
+    return [ch for ch in range(40) if abs(channel_freq_mhz(ch) - int(center_mhz)) + 1 <= 2 * int(decim)]
+
+
+def wideband_taps(decim: int, center_mhz: int, channel: int, out_shift: int = -1):
+    """The channelizer's complex int16 taps of `channel` (btle_b200_wideband_taps): (int16 [T, 2] = Re, Im; output
+    shift).  Host only: needs no GPU."""
+    L = _native.load()
+    cfg = _wideband_cfg(decim, center_mhz, out_shift)
+    n, shift = ctypes.c_size_t(0), ctypes.c_int(0)
+    rc = L.btle_b200_wideband_taps(cfg.ctypes.data, int(channel), None, 0, ctypes.byref(n), ctypes.byref(shift))
+    if rc not in (0, BTLE_EOVERFLOW):
+        raise BtleError(rc, f"no wideband taps for decim={decim}, center={center_mhz} MHz, channel={channel} "
+                            "(decim must be 2..64, the channel 0..39 and inside the band)")
+    taps = np.zeros((n.value, 2), dtype=np.int16)
+    rc = L.btle_b200_wideband_taps(cfg.ctypes.data, int(channel), taps.ctypes.data, n.value, ctypes.byref(n), ctypes.byref(shift))
+    if rc != 0:
+        raise BtleError(rc, L.btle_b200_strerror(rc).decode())
+    return taps, shift.value
 
 
 class BtleRx:
@@ -106,6 +135,66 @@ class BtleRx:
         self._check(self._L.btle_b200_rx_sps8(self._h, iq16.ctypes.data, n, int(channel), int(crc_init), int(access_addr), out.ctypes.data, cap,
                                               ctypes.byref(n_out)))
         return out[:n_out.value]
+
+    # ---- wideband captures (one capture of the band -> per-channel 4 Msps captures) --------------------------------
+    def _wide_channels(self, decim, center_mhz, channels):
+        if channels is None:
+            channels = band_channels(decim, center_mhz)
+            if len(channels) != 40:
+                raise BtleError(BTLE_EINVAL, f"a capture at {4 * decim} Msps around {center_mhz} MHz does not hold all 40 channels; "
+                                             "pass `channels`")
+        return np.ascontiguousarray(channels, dtype=np.int32).reshape(-1)
+
+    def channelize(self, wide: np.ndarray, decim: int, center_mhz: int, channels=None, out_shift: int = -1) -> np.ndarray:
+        """wide: int8 interleaved I,Q at 4 MHz * decim -> int8 [n_ch, 2 * ceil(N / decim)]: the 4 Msps captures of
+        `channels` (None = all 40, which the band must hold), e.g. for hop.follow_connections_windowed."""
+        wide = np.ascontiguousarray(wide, dtype=np.int8).reshape(-1)
+        ch = self._wide_channels(decim, center_mhz, channels)
+        n = wide.size // 2
+        width = 2 * ((n + decim - 1) // decim) if decim > 0 else 0
+        stride = (width + 15) & ~15
+        out = np.zeros((ch.size, max(stride, 16)), dtype=np.int8)
+        cfg = _wideband_cfg(decim, center_mhz, out_shift)
+        self._check(self._L.btle_b200_channelize(self._h, wide.ctypes.data, n, cfg.ctypes.data, ch.ctypes.data, ch.size,
+                                                 out.ctypes.data, out.shape[1]))
+        return np.ascontiguousarray(out[:, :width])
+
+    def channelize_device(self, d_wide, decim: int, center_mhz: int, channels, d_out, out_shift: int = -1, stream_ptr: int = 0):
+        """d_wide: torch int8 CUDA tensor (2N, interleaved I,Q); d_out: torch int8 CUDA tensor [n_ch, stride] (stride a
+        multiple of 16, >= 2 * ceil(N / decim)).  Enqueued on `stream_ptr`, not synchronised."""
+        ch = self._wide_channels(decim, center_mhz, channels)
+        assert d_out.dim() == 2 and d_out.shape[0] == ch.size and d_out.stride(1) == 1
+        cfg = _wideband_cfg(decim, center_mhz, out_shift)
+        self._check(self._L.btle_b200_channelize_device(self._h, d_wide.data_ptr(), d_wide.numel() // 2, cfg.ctypes.data, ch.ctypes.data,
+                                                        ch.size, d_out.data_ptr(), d_out.stride(0), ctypes.c_void_p(stream_ptr)))
+
+    def rx_wideband(self, wide, decim: int, center_mhz: int, cfgs: np.ndarray, cap: int | None = None) -> np.ndarray:
+        """Channelize `wide` (numpy int8, or a page-locked torch CPU tensor) and decode channel cfgs[i]["channel"] as
+        stream i, in one receiver launch (btle_b200_rx_wideband)."""
+        if hasattr(wide, "data_ptr"):
+            assert wide.dtype.itemsize == 1 and wide.is_contiguous() and not wide.is_cuda
+            ptr, n = wide.data_ptr(), wide.numel() // 2
+        else:
+            wide = np.ascontiguousarray(wide, dtype=np.int8).reshape(-1)
+            ptr, n = wide.ctypes.data, wide.size // 2
+        cfgs = np.ascontiguousarray(cfgs, dtype=CFG_DTYPE).reshape(-1)
+        cfg = _wideband_cfg(decim, center_mhz)
+        m = (n + decim - 1) // decim if decim > 0 else 0
+        grow = cap is None
+        if cap is None:
+            cap = cfgs.size * (2 * m // 16384) * 34 + 16
+        while True:
+            out = np.empty(cap, dtype=REC_DTYPE)
+            n_out = ctypes.c_size_t(0)
+            rc = self._L.btle_b200_rx_wideband(self._h, ptr, n, cfg.ctypes.data, cfgs.ctypes.data, cfgs.size, out.ctypes.data, cap,
+                                               ctypes.byref(n_out))
+            if rc == BTLE_EOVERFLOW and grow:
+                cap, grow = n_out.value, False
+                continue
+            if rc == BTLE_EOVERFLOW:
+                raise BtleError(rc, f"{n_out.value} packets found, capacity {cap}")
+            self._check(rc)
+            return out[:n_out.value]
 
     # ---- unbounded capture, pushed in pieces (btle_b200_stream_*) -----------------------------
     def stream(self, segment_chunks: int = 0, **cfg) -> "RxStream":

@@ -339,3 +339,35 @@ def channel_plan(n_streams: int, rssi: int = 0) -> np.ndarray:
     c["access_addr"] = np.where(adv, ADV_ACCESS_ADDR, 0x60850A1B + ch).astype(np.uint32)
     c["crc_init"] = np.where(adv, ADV_CRC_INIT, 0xA77B22 ^ ch).astype(np.uint32)
     return c
+
+
+def wideband_from_channels(caps, channels, decim: int, center_mhz: int, noise: float = 0.0, seed: int = 0, device=None):
+    """One int8 interleaved I,Q capture at 4 MHz * decim centred on center_mhz that carries per-channel 4 Msps captures
+    caps [n_ch, 2M] (int8, M a multiple of 4) on `channels`: each is band-limited to +-1 MHz in the FFT domain, placed at
+    bin offset q*M/4 (q = f_ch - fc in MHz) of an N = M*decim point spectrum, so that wideband sample m*decim carries
+    sample m of the channel; then the inverse FFT, seeded Gaussian noise of `noise` LSB per component, rounding and
+    clipping.  Deliberately independent of the library's channelizer taps.  torch only; runs on `device` (CPU default).
+    Returns an int8 tensor of 2N values."""
+    from .hop import channel_freq_mhz
+    dev = torch.device(device) if device is not None else torch.device("cpu")
+    caps = torch.as_tensor(np.ascontiguousarray(caps, dtype=np.int8) if not torch.is_tensor(caps) else caps).to(dev)
+    caps = caps.reshape(len(channels), -1)
+    m = caps.shape[1] // 2
+    assert m % 4 == 0, "channel captures must hold a multiple of 4 samples"
+    n = m * decim
+    spec = torch.zeros(n, dtype=torch.complex128, device=dev)
+    k = torch.fft.fftfreq(m, d=1.0 / m, device=dev).round().to(torch.int64)          # signed bin index
+    keep = k.abs() <= m // 4                                                          # |f| <= 1 MHz
+    for i, ch in enumerate(channels):
+        q = channel_freq_mhz(int(ch)) - int(center_mhz)
+        assert abs(q) + 1 <= 2 * decim, f"channel {ch} is outside the band"
+        x = caps[i].to(torch.float64).reshape(m, 2)
+        xs = torch.fft.fft(torch.complex(x[:, 0], x[:, 1]))
+        spec.index_add_(0, (k[keep] + q * m // 4) % n, xs[keep] * decim)
+    w = torch.fft.ifft(spec)
+    out = torch.stack([w.real, w.imag], dim=1)
+    if noise:
+        gen = torch.Generator(device=dev)
+        gen.manual_seed(seed)
+        out = out + noise * torch.randn(out.shape, generator=gen, device=dev, dtype=torch.float64)
+    return torch.clamp(torch.round(out), -128, 127).to(torch.int8).reshape(-1)

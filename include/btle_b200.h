@@ -296,6 +296,42 @@ int btle_b200_ber_run(btle_b200_ctx *ctx, const btle_ber_cfg *cfg, size_t n_pack
 int btle_b200_rx_iq16(btle_b200_ctx *ctx, const int16_t *iq16, size_t n_int16, int shift, const btle_stream_cfg *cfg,
                       btle_pkt_rec *out, size_t cap, size_t *n_out);
 
+/* ---- wideband captures: exact integer channelizer (DESIGN.md §6.5) ------------------------------------------------
+ * Input: ONE capture of n_samples complex samples, int8 interleaved I,Q (hackrf_transfer -r, UHD sc8) at
+ * fs = 4 MHz * decim, centred on center_mhz.  Channel ch (f_ch = btle_b200_get_freq_by_channel_number(ch), offset
+ * q = (f_ch - fc) / 1 MHz) is inside the band iff |q| + 1 <= fs/2 / 1 MHz.  For each output sample m < ceil(N / decim),
+ * with x[n] = 0 outside [0, N) and c = (T-1)/2:
+ *   acc[m] = sum_{t<T} x[m*decim + c - t] * H_q[t]                       complex, int32 (no overflow is possible)
+ *   rot[m] = acc[m] * (-j)^((q*m) mod 4)                                  exact swap / negate of the int32 pair
+ *   y[m]   = sat8((rot[m] + 2^(s-1)) >> s)  per component                 arithmetic shift, s = 0: no rounding term
+ * H_q[t] = round(G * h[t] * exp(+j*2*pi*q*(t-c)/(4*decim))), h one odd-length, symmetric, real low-pass prototype per
+ * decim (>= 50 dB from 1.25 MHz off the channel centre to fs/2, <= 1 dB droop within 0.6 MHz).  y is the channel at
+ * 4 Msps with no delay: output sample m is wideband sample decim*m, so a record at (chunk, n0) lies at wideband sample
+ * decim * (8192*chunk + n0).  Output layout [n_ch][out_stride_int8] int8 I,Q: the receiver's input format. */
+typedef struct {
+  int32_t decim;         /* 2..64: fs = 4 MHz * decim                                                           */
+  int32_t center_mhz;    /* centre frequency of the capture, whole MHz                                          */
+  int32_t out_shift;     /* -1 = default s (passband gain 1: output LSB = input LSB), else 0..31               */
+  int32_t reserved;
+} btle_wideband_cfg;
+/* Host only (no context, no GPU): the T complex taps H_q[t] of `channel` as taps[2t] = Re, taps[2t+1] = Im, and the
+ * shift `cfg` selects.  *n_taps = T always; BTLE_EOVERFLOW if cap (in complex taps) < T. */
+int btle_b200_wideband_taps(const btle_wideband_cfg *cfg, int channel, int16_t *taps, size_t cap, size_t *n_taps,
+                            int *out_shift);
+/* Device buffers: d_wide (16-byte aligned, 2*n_samples int8) -> d_out (16-byte aligned) row i = channels[i] (host
+ * array; duplicates allowed), out_stride_int8 a multiple of 16 and >= 2*ceil(n_samples/decim).  Enqueued on
+ * cuda_stream, not synchronised. */
+int btle_b200_channelize_device(btle_b200_ctx *ctx, const int8_t *d_wide, size_t n_samples, const btle_wideband_cfg *cfg,
+                                const int32_t *channels, size_t n_ch, int8_t *d_out, size_t out_stride_int8, void *cuda_stream);
+/* The same with host buffers (wide page-locked or pageable; out pageable is fine); returns when `out` is filled. */
+int btle_b200_channelize(btle_b200_ctx *ctx, const int8_t *wide, size_t n_samples, const btle_wideband_cfg *cfg,
+                         const int32_t *channels, size_t n_ch, int8_t *out, size_t out_stride_int8);
+/* Channelize into context-owned scratch, then the receiver over all channels in one launch: channel i is
+ * cfgs[i].channel, its records carry stream = i.  == btle_b200_rx_batch() over btle_b200_channelize()'s output
+ * (n_int8 = 2*ceil(n_samples/decim) per channel), record for record; BTLE_EOVERFLOW as there. */
+int btle_b200_rx_wideband(btle_b200_ctx *ctx, const int8_t *wide, size_t n_samples, const btle_wideband_cfg *cfg,
+                          const btle_stream_cfg *cfgs, size_t n_ch, btle_pkt_rec *out, size_t cap, size_t *n_out);
+
 /* ---- packet synthesiser (SURVEY.md §8f-1): the transmit PHY as a GPU kernel ---------------------
  * Integer GFSK modulation of n_packets packets given as air bytes (preamble, access address,
  * whitened PDU+CRC; bits LSB first), d_air [n_packets][max_bytes], d_nbytes [n_packets].
